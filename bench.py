@@ -346,16 +346,35 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+def dump_humans(out_dir, prefix, humans, cap):
+    """the human_t records a caller of the timed path receives for one batch (`humans`: one HUMAN_DT array per frame), as
+    float32 arrays: <prefix>_human_parts.npy [N, cap, 18, 4] (has_value, x, y, score of every part), <prefix>_human_scores.npy
+    [N, cap], both zero past a frame's count, and <prefix>_human_counts.npy [N].
+    The timed path copies seeded synthetic conf / PAF tensors over the backbone's outputs (set_output_override), so these records
+    depend on the parse stage alone: equal dumps from two builds say nothing about their conv kernels (tests/test_engine_gpu.py
+    compares those with a PyTorch reference)."""
+    os.makedirs(out_dir, exist_ok=True)
+    parts = np.zeros((len(humans), cap, 18, 4), np.float32)
+    scores = np.zeros((len(humans), cap), np.float32)
+    for i, h in enumerate(humans):
+        p = h["parts"]
+        parts[i, :len(h)] = np.stack([p["has_value"], p["x"], p["y"], p["score"]], axis=-1)
+        scores[i, :len(h)] = h["score"]
+    np.save(os.path.join(out_dir, f"{prefix}_human_parts.npy"), parts)
+    np.save(os.path.join(out_dir, f"{prefix}_human_scores.npy"), scores)
+    np.save(os.path.join(out_dir, f"{prefix}_human_counts.npy"), np.array([len(h) for h in humans], np.float32))
+
+
 # ------------------------------------------------------------------------------------------------
 def measure(args, key, dist_ctx, headline=True):
-    """one workload on this rank's GPU; returns (on rank 0) the JSON-line dict.  headline=False: a shorter run for the
-    `extra_configs` entries (no CPU baseline, no parse-batch sweep)."""
+    """one workload on this rank's GPU; returns (on rank 0) the JSON-line dict.  headline=False: the `extra_configs` entries
+    (shorter pre-load, no CPU baseline, no parse-batch sweep)."""
     import torch
     import torch.distributed as dist
     from hyperpose_b200 import capi, models, synthetic as syn
     select_workload(key)
     rank, local_rank, world, dev = dist_ctx
-    steps = args.steps if headline else max(10, min(args.steps, 20))
+    steps = args.steps
     warmup = args.warmup
 
     graph = getattr(models, WL["graph"])(seed=0)
@@ -457,6 +476,7 @@ def measure(args, key, dist_ctx, headline=True):
         if dpend["t"] is not None:
             h = engine.collect_pose(dpend["t"], cap=HCAP)
             dpend["t"] = None
+            dpend["last"] = h
             return h
 
     # e2e: the public host call, pinned host frames in, human_t records out -- two batches in flight
@@ -551,6 +571,8 @@ def measure(args, key, dist_ctx, headline=True):
     # pass A: the timed K steps, per-op profiling OFF -> value
     ms_total, launches = timed(step_device, steps, warmup)
     clocks = sampler.stop() if rank == 0 and headline else None
+    if args.dump_outputs and rank == 0:
+        dump_humans(args.dump_outputs, f"{key}_{args.dtype}", dpend.pop("last") if use_graph else parser.fetch(BATCH, cap=HCAP), HCAP)
     # pass B: the same K steps with per-op CUDA events on the launching stream -> kernel time for the roofline
     saved_graph = use_graph
     use_graph = False                       # per-op events need the kernels launched one by one
@@ -672,9 +694,10 @@ def measure(args, key, dist_ctx, headline=True):
         layers = [{"op": i, "name": graph.ops[i].name, "type": int(prof_ty[i]), "ms": float(prof_ms[i]),
                    "tflops": (float(prof_fl[i]) * BATCH / (prof_ms[i] / 1e3) / 1e12 if prof_ms[i] > 0 and prof_fl[i] > 0 else None)}
                   for i in range(len(prof_ms))]
-        os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-        with open(os.path.join(ROOT, "gpurun_out", f"bench_layers_{key}_{args.dtype}_n{world}.json"), "w") as f:
-            json.dump({"ms_per_step": ms_total / steps, "conv_ms": conv_ms, "other_engine_ms": other_ms, "profiled_runs": prof_runs, "layers": layers}, f, indent=1)
+        if args.layers_dir:
+            os.makedirs(args.layers_dir, exist_ok=True)
+            with open(os.path.join(args.layers_dir, f"bench_layers_{key}_{args.dtype}_n{world}.json"), "w") as f:
+                json.dump({"ms_per_step": ms_total / steps, "conv_ms": conv_ms, "other_engine_ms": other_ms, "profiled_runs": prof_runs, "layers": layers}, f, indent=1)
         # bounded CPU baseline (rank 0, N=1, headline only): the reference parser on the host cores + the conv port
         if world == 1 and headline and not args.no_cpu_baseline and not PIFPAF:
             cores = cpu_threads()
@@ -756,6 +779,9 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the extra_configs entries (cfg2 / cfg4 / cfg5) of the default run")
     ap.add_argument("--no-tf32-line", action="store_true", help="skip the tf32 entry of the default run")
     ap.add_argument("--workload", default="cfg3", choices=sorted(WORKLOADS), help="BASELINE.json config (default: the headline cfg3)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the keypoint records of the last timed step of every measured config to "
+                    "DIR/<config>_<dtype>_human_*.npy; they come from the synthetic parser inputs, not from the convs (see dump_humans)")
+    ap.add_argument("--layers-dir", metavar="DIR", help="write the per-op CUDA-event times of every measured config to DIR/bench_layers_*.json")
     args = ap.parse_args()
     select_workload(args.workload)
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup

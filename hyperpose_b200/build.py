@@ -9,6 +9,9 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libhyperpose_b200.so")
+# binaries compiled from the drop-in together with the reference's headers / sources: kept out of git with the reference's builds,
+# in a directory of their own (the rest of oracle/_ref is the checker, built from the reference alone by oracle/Makefile)
+REF_BIN = os.path.join(ROOT, "oracle", "_ref", "dropin")
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC,-O2,-Wall", "-Xptxas", "-v"]
@@ -68,16 +71,17 @@ def build(force: bool = False, verbose: bool = False) -> str:
 def build_cpp_example(ref_root: str = "/root/reference") -> str | None:
     """Compiles the C++ drop-in (hyperpose_api/*.cpp) + examples/operator_api_b200.cpp against the reference's
     UNCHANGED public headers.  Needs the reference tree (headers are not copied into this repo); returns the
-    binary path, or None when the reference is absent (GPU box: the prebuilt binary travels with the snapshot)."""
-    exe = os.path.join(ROOT, "examples", "operator_api_b200")
+    binary path (oracle/_ref/dropin/operator_api_b200), or the one built earlier / None when the reference is absent."""
+    exe = os.path.join(REF_BIN, "operator_api_b200")
     if not os.path.isdir(os.path.join(ref_root, "include", "hyperpose")):
         return exe if os.path.exists(exe) else None
+    os.makedirs(REF_BIN, exist_ok=True)
     api = os.path.join(CSRC, "hyperpose_api")
     srcs = [os.path.join(api, "paf.cpp"), os.path.join(api, "tensorrt.cpp"), os.path.join(api, "pifpaf.cpp"), os.path.join(api, "pose_proposal.cpp"),
             os.path.join(ROOT, "examples", "operator_api_b200.cpp")]
     if _newer(srcs + [LIB], exe):
         cmd = ["g++", "-std=c++17", "-O2", "-DHP_B200_STANDALONE", "-I" + os.path.join(CSRC, "shim"), "-I" + os.path.join(ref_root, "include"),
-               "-I" + os.path.join(ROOT, "include")] + srcs + ["-L" + PKG, "-lhyperpose_b200", "-Wl,-rpath,$ORIGIN/../hyperpose_b200", "-o", exe]
+               "-I" + os.path.join(ROOT, "include")] + srcs + ["-L" + PKG, "-lhyperpose_b200", "-Wl,-rpath,$ORIGIN/../../../hyperpose_b200", "-o", exe]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode:
             sys.stderr.write(r.stdout + r.stderr)
@@ -89,9 +93,10 @@ def build_stream_example(ref_root: str = "/root/reference", mock: bool = False) 
     """examples/stream_api_b200.cpp: the reference's STREAM API on the drop-in.  The scheduler is the reference's own --
     include/hyperpose/stream/stream.hpp instantiated as it is, src/stream.cpp + src/thread_pool.cpp + src/logging.cpp compiled from
     the reference tree unchanged.  mock=True builds the CPU self-check variant (stand-in engine / parser, no GPU, no library)."""
-    exe = os.path.join(ROOT, "examples", "stream_api_b200_mock" if mock else "stream_api_b200")
+    exe = os.path.join(REF_BIN, "stream_api_b200_mock" if mock else "stream_api_b200")
     if not os.path.isdir(os.path.join(ref_root, "include", "hyperpose")):
         return exe if os.path.exists(exe) else None
+    os.makedirs(REF_BIN, exist_ok=True)
     api = os.path.join(CSRC, "hyperpose_api")
     ref = [os.path.join(ref_root, "src", f) for f in ("stream.cpp", "thread_pool.cpp", "logging.cpp")]
     srcs = [os.path.join(ROOT, "examples", "stream_api_b200.cpp")] + ref
@@ -101,7 +106,7 @@ def build_stream_example(ref_root: str = "/root/reference", mock: bool = False) 
         cmd = ["g++", "-std=c++17", "-O2", "-pthread", "-DHP_STREAM_MOCK" if mock else "-DHP_B200_STANDALONE", "-I" + os.path.join(CSRC, "shim"),
                "-I" + os.path.join(ref_root, "include"), "-I" + os.path.join(ref_root, "src"), "-I" + os.path.join(ROOT, "include")] + srcs
         if not mock:
-            cmd += ["-L" + PKG, "-lhyperpose_b200", "-Wl,-rpath,$ORIGIN/../hyperpose_b200"]
+            cmd += ["-L" + PKG, "-lhyperpose_b200", "-Wl,-rpath,$ORIGIN/../../../hyperpose_b200"]
         cmd += ["-o", exe]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode:
@@ -119,8 +124,8 @@ def build_reference_examples(ref_root: str = "/root/reference") -> dict | None:
     the reference's unchanged headers, its unchanged src/{stream,thread_pool,logging,human,data}.cpp (scheduler, drawing, batching
     helpers), the B200 classes of hyperpose_api/*.cpp underneath, and the OpenCV / gflags stand-ins of csrc/shim (neither library
     exists in this image).  Nothing of the reference is copied: every source is compiled where it lies.  Returns {name: binary} in
-    examples/ref_build/ (git-ignored, travels to the GPU box), or the prebuilt set / None where the reference tree is absent."""
-    out_dir = os.path.join(ROOT, "examples", "ref_build")
+    oracle/_ref/dropin/ref_build/, or the set built earlier / None where the reference tree is absent."""
+    out_dir = os.path.join(REF_BIN, "ref_build")
     exes = {n: os.path.join(out_dir, n.replace(".example", "")) for n in REFERENCE_EXAMPLES}
     if not os.path.isdir(os.path.join(ref_root, "include", "hyperpose")):
         return exes if all(os.path.exists(e) for e in exes.values()) else None
@@ -145,7 +150,7 @@ def build_reference_examples(ref_root: str = "/root/reference") -> dict | None:
     for name, exe in exes.items():
         src = os.path.join(ref_root, "examples", name + ".cpp")
         if _newer([src, LIB] + objs, exe):
-            cmd = ["g++", "-std=c++17", "-O2", "-pthread"] + inc + [src] + objs + ["-L" + PKG, "-lhyperpose_b200", "-Wl,-rpath,$ORIGIN/../../hyperpose_b200", "-o", exe]
+            cmd = ["g++", "-std=c++17", "-O2", "-pthread"] + inc + [src] + objs + ["-L" + PKG, "-lhyperpose_b200", "-Wl,-rpath,$ORIGIN/../../../../hyperpose_b200", "-o", exe]
             r = subprocess.run(cmd, capture_output=True, text=True)
             if r.returncode:
                 sys.stderr.write(r.stdout + r.stderr)

@@ -11,6 +11,8 @@
 2. ref_humans.npz  -- human_t lists produced by the reference's OWN src/paf.cpp (compiled
                       verbatim into oracle/_ref by oracle/Makefile) on the seeded synthetic
                       frames of hyperpose_b200/synthetic.py (SURVEY 8d configs).
+3. ref_live.npz    -- (`python tests/golden/make_golden.py live`) the reference parsers' outputs
+                      on the random / sweep inputs of the tests that compare against them.
 """
 import hashlib
 import os
@@ -71,6 +73,97 @@ AREA_FRAME_CASES = [
     ("user_frac", 15, 3, 46, 54, 41, 33, 0.05, 0.05),        # fractional reduction on both axes
     ("user_keep_x", 16, 3, 46, 54, 54, 30, 0.05, 0.05),      # one axis kept (scale 1), the other shrinks: area regime
 ]
+
+
+def random_case(seed):
+    """frame of test_oracle_matches_live_reference_random: (conf, paf)"""
+    rng = np.random.default_rng(seed)
+    hf, wf = [(46, 54), (46, 82), (32, 32), (23, 40)][seed % 4]
+    P = int(rng.integers(0, 16))
+    from hyperpose_b200 import synthetic as syn
+    return syn.make_frame_tensors(seed, P, hf, wf)
+
+
+def noise_case():
+    """structureless input (many spurious peaks, few/no humans): (conf, paf)"""
+    rng = np.random.default_rng(99)
+    conf = rng.random((19, 24, 30), dtype=np.float32) * 0.3
+    paf = (rng.random((38, 24, 30), dtype=np.float32) - 0.5)
+    return conf, paf
+
+
+def sweep_case(seed):
+    """frame and parser settings of test_oracle_matches_live_reference_sweep: (conf, paf, ct, pt, rw, rh)"""
+    from hyperpose_b200 import synthetic as syn
+    rng = np.random.default_rng(seed)
+    hf = int(rng.integers(9, 50))
+    wf = int(rng.integers(9, min(90, 4 * hf) + 1))
+    P = int(rng.integers(0, 13))
+    noise = float(rng.choice([0.005, 0.02, 0.06]))
+    conf, paf = syn.make_frame_tensors(seed, P, hf, wf, noise=noise)
+    ct, pt = float(rng.choice([0.05, 0.1, 0.3])), float(rng.choice([0.02, 0.05, 0.2]))
+    if seed % 3 == 0:      # user resolution (w, h) >= the feature map
+        rw, rh = int(hf * rng.uniform(1.0, 4.6)) + 1, int(wf * rng.uniform(1.0, 4.6)) + 1
+        rw, rh = max(rw, wf), max(rh, hf)
+    else:
+        rw = rh = -1
+    return conf, paf, ct, pt, rw, rh
+
+
+RANDOM_SEEDS, SWEEP_SEEDS = range(20, 32), range(100, 140)
+PPN_RANDOM_ITERS = 40
+
+
+def ppn_random_case(it, rng):
+    """iteration `it` of test_restatement_vs_live_reference_random (rng: default_rng(7), advanced once per iteration)"""
+    from hyperpose_b200 import synthetic as syn
+    thr = [(0.10, 0.05, 0.3), (0.06, 0.03, 0.2), (0.2, 0.1, 0.6), (0.10, 0.05, 0.05)][it % 4]
+    return syn.make_ppn_tensors(1000 + it, (0, 8), distractors=int(rng.integers(0, 80))), thr
+
+
+def pifpaf_batch_case():
+    """the 8 frames of test_gpu_decoder_batched_vs_live_reference: (pif [8,17,5,49,49], paf [8,19,9,49,49])"""
+    from hyperpose_b200 import synthetic as syn
+    fields = [syn.make_pifpaf_fields(100 + i, (1, 9), 49, 49) for i in range(8)]
+    return np.stack([f[0] for f in fields]), np.stack([f[1] for f in fields])
+
+
+def pifpaf_handoff_case():
+    """the 2 frames of test_pifpaf_fields_hand_off: (pif [2,17,5,49,49], paf [2,19,9,49,49])"""
+    from hyperpose_b200 import synthetic as syn
+    fields = [syn.make_pifpaf_fields(20 + i, (2, 3), 49, 49) for i in range(2)]
+    return np.stack([f[0] for f in fields]).astype(np.float32), np.stack([f[1] for f in fields]).astype(np.float32)
+
+
+def make_live():
+    """tests/golden/ref_live.npz: what the reference's own parsers (oracle/_ref) return on the inputs of the tests that compare
+    against them, so that those comparisons run where the reference sources are absent"""
+    import oracle
+    assert oracle.ref_available() and oracle.pifpaf_ref_available() and oracle.ppn_ref_available()
+    out = {}
+
+    def paf_entry(key, conf, paf, ct=0.05, pt=0.05, rw=-1, rh=-1):
+        rp = oracle.RefParser(ct, pt, rw, rh)
+        out[key + "_humans"] = rp.process(conf, paf)
+        out[key + "_in_sha"] = np.array(sha(conf) + sha(paf))
+        rp.close()
+
+    for seed in RANDOM_SEEDS:
+        paf_entry(f"random{seed}", *random_case(seed))
+    paf_entry("noise", *noise_case())
+    for seed in SWEEP_SEEDS:
+        paf_entry(f"sweep{seed}", *sweep_case(seed))
+    rng = np.random.default_rng(7)
+    for it in range(PPN_RANDOM_ITERS):
+        t, thr = ppn_random_case(it, rng)
+        out[f"ppn_random{it}_humans"] = oracle.ref_ppn_process(*t, 384, 384, *thr)
+        out[f"ppn_random{it}_in_sha"] = np.array("".join(sha(a) for a in t))
+    for key, (pif, paf) in (("pp_batch", pifpaf_batch_case()), ("pp_handoff", pifpaf_handoff_case())):
+        for i in range(len(pif)):
+            out[f"{key}{i}_humans"] = oracle.ref_pifpaf_process(pif[i], paf[i], 385, 385, 0.1)
+        out[key + "_in_sha"] = np.array(sha(pif) + sha(paf))
+    np.savez_compressed(os.path.join(HERE, "ref_live.npz"), **out)
+    print({k: len(v) for k, v in out.items() if k.endswith("_humans")})
 
 
 def make_area():
@@ -167,6 +260,10 @@ def make_ppn():
 
 if __name__ == "__main__" and "area" in sys.argv[1:]:
     make_area()
+    sys.exit(0)
+
+if __name__ == "__main__" and "live" in sys.argv[1:]:
+    make_live()
     sys.exit(0)
 
 if __name__ == "__main__":

@@ -7,6 +7,7 @@ with every tensor crossing host memory.  The drop-in keeps the interface; these 
     results byte-identical to the oracle and to the ordinary host path;
   * anything else -- a copy at another address, ANY changed byte, a publication older than 4 batches, the switch
     turned off -- takes the host path and gives the same answer."""
+import os
 import threading
 
 import numpy as np
@@ -14,6 +15,7 @@ import pytest
 
 import oracle
 from hyperpose_b200 import capi, models, synthetic as syn
+from tests.golden.make_golden import pifpaf_handoff_case, sha
 
 pytestmark = pytest.mark.gpu
 
@@ -162,15 +164,14 @@ def test_stream_style_parser_replicas_on_threads():
     eng.close()
 
 
-@pytest.mark.skipif(not oracle.pifpaf_ref_available(), reason="reference decoder (oracle/_ref) not built")
-def test_pifpaf_fields_hand_off():
+def test_pifpaf_fields_hand_off(golden_dir):
     import torch
     N, HW = 2, 385
     eng = capi.Engine(models.resnet50_pifpaf(0).to_pack(), (HW, HW), max_batch_size=N)
     assert eng.head_type == 1 and (eng.out_h, eng.out_w) == (49, 49)
-    fields = [syn.make_pifpaf_fields(20 + i, (2, 3), 49, 49) for i in range(N)]
-    pif = np.stack([f[0] for f in fields]).astype(np.float32)
-    paf = np.stack([f[1] for f in fields]).astype(np.float32)
+    live = np.load(os.path.join(golden_dir, "ref_live.npz"))      # what the reference decoder (oracle/_ref) returned on these fields
+    pif, paf = pifpaf_handoff_case()
+    assert sha(pif) + sha(paf) == str(live["pp_handoff_in_sha"]), "synthetic generator drifted from the goldens"
     dp, da = torch.from_numpy(pif).cuda(), torch.from_numpy(paf).cuda()
     torch.cuda.synchronize()
     eng.set_output_override(dp.data_ptr(), da.data_ptr())
@@ -182,7 +183,9 @@ def test_pifpaf_fields_hand_off():
     for i in range(N):
         assert packets[i][0].shape == (17, 5, 49, 49) and packets[i][0].tobytes() == pif[i].tobytes()
         got = dec.process(packets[i][0], packets[i][1])
-        want = oracle.ref_pifpaf_process(pif[i], paf[i], HW, HW, 0.1)
+        want = live[f"pp_handoff{i}_humans"]
+        if oracle.pifpaf_ref_available():
+            assert oracle.ref_pifpaf_process(pif[i], paf[i], HW, HW, 0.1).tobytes() == want.tobytes()
         assert got.tobytes() == want.tobytes(), (i, len(got), len(want))
         total += len(got)
     d = _delta(s0)

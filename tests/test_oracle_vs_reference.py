@@ -1,7 +1,8 @@
 """The oracle restatement (oracle/paf_oracle.c) against the reference's OWN parser:
   * committed goldens: human_t lists that /root/reference/src/paf.cpp (compiled verbatim
     into oracle/_ref) produced on the seeded synthetic frames -- runs anywhere;
-  * live oracle/_ref, when it is built (build container, or prebuilt .so on the GPU box)."""
+  * random / noise / sweep inputs: what oracle/_ref returned on them (committed as ref_live.npz), and the live oracle/_ref
+    as well where it is built."""
 import os
 
 import numpy as np
@@ -9,12 +10,18 @@ import pytest
 
 import oracle
 from hyperpose_b200 import synthetic as syn
-from tests.golden.make_golden import AREA_FRAME_CASES, FRAME_CASES, sha
+from tests.golden.make_golden import (AREA_FRAME_CASES, FRAME_CASES, RANDOM_SEEDS, SWEEP_SEEDS, noise_case, random_case, sha,
+                                      sweep_case)
 
 
 @pytest.fixture(scope="module")
 def ref_humans(golden_dir):
     return np.load(os.path.join(golden_dir, "ref_humans.npz"))
+
+
+@pytest.fixture(scope="module")
+def live(golden_dir):
+    return np.load(os.path.join(golden_dir, "ref_live.npz"))
 
 
 @pytest.mark.parametrize("case", FRAME_CASES, ids=[c[0] for c in FRAME_CASES])
@@ -53,30 +60,27 @@ def test_goldens_are_not_vacuous(ref_humans):
     assert int(h["parts"]["has_value"].sum()) == 18
 
 
-@pytest.mark.skipif(not oracle.ref_available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("seed", range(20, 32))
-def test_oracle_matches_live_reference_random(seed):
-    rng = np.random.default_rng(seed)
-    hf, wf = [(46, 54), (46, 82), (32, 32), (23, 40)][seed % 4]
-    P = int(rng.integers(0, 16))
-    conf, paf = syn.make_frame_tensors(seed, P, hf, wf)
-    rp = oracle.RefParser()
-    want = rp.process(conf, paf)
-    rp.close()
-    got = oracle.oracle_process(conf, paf)["humans"]
-    assert got.tobytes() == want.tobytes()
+def _vs_reference(live, key, conf, paf, ct=0.05, pt=0.05, rw=-1, rh=-1):
+    """(oracle humans, reference humans): the reference's output stored in ref_live.npz, held equal to the live oracle/_ref
+    where that is built"""
+    assert sha(conf) + sha(paf) == str(live[key + "_in_sha"]), "synthetic generator drifted from the goldens"
+    want = live[key + "_humans"]
+    if oracle.ref_available():
+        rp = oracle.RefParser(ct, pt, rw, rh)
+        assert rp.process(conf, paf).tobytes() == want.tobytes()
+        rp.close()
+    return oracle.oracle_process(conf, paf, ct, pt, rw, rh), want
 
 
-@pytest.mark.skipif(not oracle.ref_available(), reason="oracle/_ref not built")
-def test_oracle_matches_live_reference_noise_field():
+@pytest.mark.parametrize("seed", RANDOM_SEEDS)
+def test_oracle_matches_live_reference_random(live, seed):
+    o, want = _vs_reference(live, f"random{seed}", *random_case(seed))
+    assert o["humans"].tobytes() == want.tobytes()
+
+
+def test_oracle_matches_live_reference_noise_field(live):
     # structureless input (many spurious peaks, few/no humans): exercises the candidate filter
-    rng = np.random.default_rng(99)
-    conf = rng.random((19, 24, 30), dtype=np.float32) * 0.3
-    paf = (rng.random((38, 24, 30), dtype=np.float32) - 0.5)
-    rp = oracle.RefParser()
-    want = rp.process(conf, paf)
-    rp.close()
-    o = oracle.oracle_process(conf, paf)
+    o, want = _vs_reference(live, "noise", *noise_case())
     assert len(o["peaks"]) > 50
     assert o["humans"].tobytes() == want.tobytes()
 
@@ -89,9 +93,8 @@ def test_peak_ids_are_scan_ordered():
     assert np.all(np.diff(key) > 0)
 
 
-@pytest.mark.skipif(not oracle.ref_available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("seed", range(100, 140))
-def test_oracle_matches_live_reference_sweep(seed):
+@pytest.mark.parametrize("seed", SWEEP_SEEDS)
+def test_oracle_matches_live_reference_sweep(live, seed):
     """wider sweep of what pins the oracle: odd feature sizes, both thresholds, custom parser resolutions (non-integer
     up-scaling factors -> the 2-tap INTER_AREA path), empty frames and crowds, noise levels around the thresholds.
     Two regions are left out because the reference itself leaves them open, not because the restatement differs:
@@ -101,20 +104,7 @@ def test_oracle_matches_live_reference_sweep(seed):
         limbs assigned differently among equal-score candidates);
       * feature maps wider than 4:1 (the default resolution then shrinks an axis) are covered separately by
         test_oracle_matches_reference_golden_on_shrinking_resolutions."""
-    rng = np.random.default_rng(seed)
-    hf = int(rng.integers(9, 50))
-    wf = int(rng.integers(9, min(90, 4 * hf) + 1))
-    P = int(rng.integers(0, 13))
-    noise = float(rng.choice([0.005, 0.02, 0.06]))
-    conf, paf = syn.make_frame_tensors(seed, P, hf, wf, noise=noise)
-    ct, pt = float(rng.choice([0.05, 0.1, 0.3])), float(rng.choice([0.02, 0.05, 0.2]))
-    if seed % 3 == 0:      # user resolution (w, h) >= the feature map
-        rw, rh = int(hf * rng.uniform(1.0, 4.6)) + 1, int(wf * rng.uniform(1.0, 4.6)) + 1
-        rw, rh = max(rw, wf), max(rh, hf)
-    else:
-        rw = rh = -1
-    rp = oracle.RefParser(ct, pt, rw, rh)
-    want = rp.process(conf, paf)
-    rp.close()
-    got = oracle.oracle_process(conf, paf, ct, pt, rw, rh)["humans"]
-    assert got.tobytes() == want.tobytes(), (hf, wf, P, noise, ct, pt, rw, rh, len(got), len(want))
+    conf, paf, ct, pt, rw, rh = sweep_case(seed)
+    o, want = _vs_reference(live, f"sweep{seed}", conf, paf, ct, pt, rw, rh)
+    got = o["humans"]
+    assert got.tobytes() == want.tobytes(), (conf.shape, ct, pt, rw, rh, len(got), len(want))

@@ -11,7 +11,7 @@ import pytest
 
 import oracle
 from hyperpose_b200 import capi, synthetic as syn
-from tests.golden.make_golden import PIFPAF_CASES, sha
+from tests.golden.make_golden import PIFPAF_CASES, pifpaf_batch_case, sha
 
 
 @pytest.fixture(scope="module")
@@ -64,15 +64,17 @@ def test_gpu_decoder_equals_reference_golden(gold, case):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not oracle.pifpaf_ref_available(), reason="oracle/_ref/libref_pifpaf.so not built")
-def test_gpu_decoder_batched_vs_live_reference():
-    N, h, w = 8, 49, 49
-    fields = [syn.make_pifpaf_fields(100 + i, (1, 9), h, w) for i in range(N)]
-    pif = np.stack([f[0] for f in fields]); paf = np.stack([f[1] for f in fields])
+def test_gpu_decoder_batched_vs_live_reference(golden_dir):
+    """against what oracle/_ref returned on these frames (ref_live.npz), and against the live oracle/_ref as well where it is built"""
+    live = np.load(os.path.join(golden_dir, "ref_live.npz"))
+    pif, paf = pifpaf_batch_case()
+    assert sha(pif) + sha(paf) == str(live["pp_batch_in_sha"]), "synthetic generator drifted from the goldens"
     dec = capi.PifPafParser(385, 385, 0.1)
     got = dec.process_batch(pif, paf)
-    for i in range(N):
-        want = oracle.ref_pifpaf_process(pif[i], paf[i], 385, 385, 0.1)
+    for i in range(len(pif)):
+        want = live[f"pp_batch{i}_humans"]
+        if oracle.pifpaf_ref_available():
+            assert oracle.ref_pifpaf_process(pif[i], paf[i], 385, 385, 0.1).tobytes() == want.tobytes()
         d = _diff(got[i], want)
         assert d is None, f"frame {i}: {d}"
     dec.close()

@@ -1,7 +1,8 @@
 """Pose Proposal Network parse path (SURVEY 8f rank 3; hyperpose::parser::pose_proposal, src/pose_proposal.cpp:68-337).
 Checker = the reference's OWN source compiled verbatim (oracle/_ref/libref_ppn.so); its outputs on seeded synthetic tensors
 are committed as tests/golden/ref_ppn.npz, and oracle/ppn_oracle.py restates the algorithm for boxes without the reference.
-  * CPU: goldens are non-vacuous, the generator reproduces their inputs, the restatement == goldens == live reference;
+  * CPU: goldens are non-vacuous, the generator reproduces their inputs, the restatement == goldens (== live reference where
+    oracle/_ref is built);
   * GPU: the CUDA parser, through the C ABI, equals the goldens and the restatement byte-for-byte."""
 import os
 
@@ -10,7 +11,7 @@ import pytest
 
 import oracle
 from hyperpose_b200 import capi, synthetic as syn
-from tests.golden.make_golden import PPN_CASES, sha
+from tests.golden.make_golden import PPN_CASES, PPN_RANDOM_ITERS, ppn_random_case, sha
 
 
 @pytest.fixture(scope="module")
@@ -70,13 +71,17 @@ def test_live_reference_matches_golden(gold, case):
     assert got.tobytes() == gold[name + "_humans"].tobytes()
 
 
-@pytest.mark.skipif(not oracle.ppn_ref_available(), reason="oracle/_ref/libref_ppn.so not built")
-def test_restatement_vs_live_reference_random():
+def test_restatement_vs_live_reference_random(golden_dir):
+    """the restatement against what oracle/_ref returned on these inputs (ref_live.npz), and against the live oracle/_ref
+    as well where it is built"""
+    live = np.load(os.path.join(golden_dir, "ref_live.npz"))
     rng = np.random.default_rng(7)
-    for it in range(40):
-        pt, lt, nt = [(0.10, 0.05, 0.3), (0.06, 0.03, 0.2), (0.2, 0.1, 0.6), (0.10, 0.05, 0.05)][it % 4]
-        t = syn.make_ppn_tensors(1000 + it, (0, 8), distractors=int(rng.integers(0, 80)))
-        want = oracle.ref_ppn_process(*t, 384, 384, pt, lt, nt)
+    for it in range(PPN_RANDOM_ITERS):
+        t, (pt, lt, nt) = ppn_random_case(it, rng)
+        assert "".join(sha(a) for a in t) == str(live[f"ppn_random{it}_in_sha"]), "synthetic generator drifted from the goldens"
+        want = live[f"ppn_random{it}_humans"]
+        if oracle.ppn_ref_available():
+            assert oracle.ref_ppn_process(*t, 384, 384, pt, lt, nt).tobytes() == want.tobytes()
         got = _as_records(oracle.ppn_process(*t, 384, 384, pt, lt, nt))
         d = _diff(got, want)
         assert d is None, f"seed {1000 + it} thr {(pt, lt, nt)}: {d}"

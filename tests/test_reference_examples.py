@@ -5,7 +5,7 @@ Build (hyperpose_b200/build.py::build_reference_examples): every source is compi
 the example, examples/utils.cpp, and the reference's own src/{stream,thread_pool,logging,human,data}.cpp (scheduler,
 draw_human, non_scaling_resize) -- over the unchanged public headers, with the B200 classes of csrc/hyperpose_api underneath
 and the OpenCV / gflags stand-ins of csrc/shim (neither library exists in this image).  The binaries land in
-examples/ref_build/ and travel to the GPU box with the snapshot.
+oracle/_ref/dropin/ref_build/, with the other builds of the reference's sources.
 
 Inputs: the shim's only image container is binary PPM, so the "images" are P6 files named *.png and the "video" is P6 frames
 back to back; model files are HPB2PACK packs named as the example expects (.onnx where it insists on that suffix)."""
@@ -18,7 +18,6 @@ import pytest
 from hyperpose_b200 import build as hb, models, synthetic as syn
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-HAVE_REF = os.path.isdir("/root/reference/include/hyperpose")
 
 
 def _p6(frame_bgr: np.ndarray) -> bytes:
@@ -50,14 +49,13 @@ def _read_p6_stream(path):
 def _exes():
     exes = hb.build_reference_examples()
     if exes is None:
-        pytest.skip("reference examples not built (need /root/reference at build time; the GPU box uses the prebuilt binaries)")
+        pytest.skip("reference examples not built (they need the reference's sources at build time)")
     return exes
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree absent")
 def test_reference_examples_build_unmodified_against_the_dropin():
-    exes = hb.build_reference_examples()
-    assert exes and len(exes) == 6
+    exes = _exes()
+    assert len(exes) == 6
     for name, exe in exes.items():
         assert os.path.exists(exe), name
     syms = subprocess.run(["nm", "-C", "--defined-only", exes["cli"]], capture_output=True, text=True).stdout
